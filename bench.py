@@ -24,6 +24,7 @@ Besides the contract's keys the line carries
              Trainer(kvstore='device'), row_sparse push + row_sparse_pull
 
 Usage: python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...]
+                       [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -713,10 +714,10 @@ def bert_base(torch, seq):
     return transformers.BertForMaskedLM(cfg)
 
 
-def train_steps(env, args, which):
-    """One JSON-able dict: samples/sec of `which` ('resnet50' | 'bert') training steps -- torch forward/backward in
-    bf16, Trainer(kvstore='device') exchanging + updating (fused, multi-precision: fp32 master weights and state
-    in the engine) every parameter in one launch per step."""
+def train_steps(env, args, which, steps, dump=None):
+    """One JSON-able dict: samples/sec of `steps` timed `which` ('resnet50' | 'bert') training steps -- torch
+    forward/backward in bf16, Trainer(kvstore='device') exchanging + updating (fused, multi-precision: fp32 master
+    weights and state in the engine) every parameter in one launch per step.  dump: --dump-outputs directory."""
     torch, mx = env.torch, env.mx
     torch.manual_seed(0)
     if which == "resnet50":
@@ -761,7 +762,7 @@ def train_steps(env, args, which):
         torch._foreach_zero_(gl)
         return loss
 
-    steps, warm = min(args.steps, 30), max(3, args.warmup)
+    warm = max(3, args.warmup)
     for _ in range(warm):
         step()
     torch.cuda.synchronize(); env.barrier()
@@ -774,6 +775,10 @@ def train_steps(env, args, which):
     e1.record()
     torch.cuda.synchronize()
     ms, comm_ms = env.max_over_ranks([e0.elapsed_time(e1) / steps, sum(a.elapsed_time(b) for a, b in ec) / steps])
+    if dump and env.rank == 0:          # before the traced step below updates the parameters again
+        mx.nd.waitall()
+        dump_outputs(dump, [("param_%03d" % i, p.numel(), lambda p=p: p.detach().float().cpu().numpy())
+                            for i, p in enumerate(params)])
     nparam = sum(p.numel() for p in params)
     # one traced step: where the buckets' exchange ran relative to backward (CUDA events on the engine stream
     # against events on the framework stream; stands in for an nsys timeline, which this image does not have)
@@ -820,7 +825,7 @@ def train_steps(env, args, which):
 # step = row_sparse push (union + gather-sum + lazy SGD-momentum on the touched rows) followed by
 # row_sparse_pull of the same ids.
 # ---------------------------------------------------------------------------
-def bench_rsp(env, args):
+def bench_rsp(env, args, steps, dump=None):
     torch, mx = env.torch, env.mx
     rank, world, ctx = env.rank, env.world, env.ctx
     R, L, nnz = 1_000_000, 256, 10_000
@@ -838,7 +843,7 @@ def bench_rsp(env, args):
         kv.push("emb", grad)
         kv.row_sparse_pull("emb", out=out, row_ids=ids)
 
-    steps, warm = min(max(args.steps, 20), 100), max(3, args.warmup)
+    warm = max(3, args.warmup)
     for _ in range(warm):
         step()
     torch.cuda.synchronize(); env.barrier()
@@ -851,6 +856,9 @@ def bench_rsp(env, args):
     torch.cuda.synchronize()
     ms = env.max_over_ranks([e0.elapsed_time(e1) / steps])[0]
     union = int(out.indices.shape[0])
+    if dump and env.rank == 0:          # the rows the last pull returned, and their row ids
+        dump_outputs(dump, [("out_data", out.data.size, out.data.asnumpy),
+                            ("out_indices", union, lambda: out.indices.asnumpy().astype(np.float64))])
     # parity of exactly this shape: the pulled rows against the oracle's lazy SGD-momentum after warm+steps pushes
     # is the job of tests/test_gpu_rsp.py::test_c5_shape; here the union size is cross-checked
     all_idx = np.unique(np.concatenate([np.sort(np.random.default_rng(1234 + r).choice(R, nnz, replace=False))
@@ -873,6 +881,38 @@ def bench_rsp(env, args):
            "gpu_launches": mx.kv.launch_count() - launches0}
     del kv
     return res
+
+
+# timed steps of the secondaries the sweep runs: fixed, so that --steps sets the headline's count alone
+SECONDARY_TRAIN_STEPS = 30
+SECONDARY_RSP_STEPS = 100
+
+DUMP_LIMIT_ELEMS = 8 << 20      # --dump-outputs writes at most 8 Mi elements (32 MiB of float32)
+
+
+def dump_counts(sizes, limit=DUMP_LIMIT_ELEMS):
+    """How many elements of each array --dump-outputs writes: every array whole while the total fits in `limit`,
+    else every array whole up to one common cap, the larger ones sampled down to it."""
+    counts, left = {}, limit
+    order = sorted(range(len(sizes)), key=lambda k: sizes[k])
+    for i, k in enumerate(order):
+        counts[k] = min(sizes[k], left // (len(order) - i))
+        left -= counts[k]
+    return [counts[k] for k in range(len(sizes))]
+
+
+def dump_outputs(path, arrays):
+    """arrays: (name, elements, fetch) per array, fetch() returning it as a numpy array.  Writes DIR/<name>.npy --
+    float64 arrays as float64, everything else as float32 -- the whole array, or (beyond the dump_counts budget) the
+    flattened array at a sorted sample of positions drawn with seed <index in arrays>, so that two runs with the same
+    arguments write the same positions."""
+    os.makedirs(path, exist_ok=True)
+    counts = dump_counts([n for _, n, _ in arrays])
+    for k, ((name, n, fetch), c) in enumerate(zip(arrays, counts)):
+        a = fetch()
+        if c < n:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(k).choice(n, c, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
 
 
 _PEAKS = None
@@ -914,7 +954,16 @@ def main():
     ap.add_argument("--local-world", type=int, default=0,
                     help="split the box into 'nodes' of this many GPUs and use kv.create('dist_device_sync'): NVLink "
                          "peer memory inside a node, NCCL between nodes (not the driver's configuration)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned, to compare two builds: the pulled weights "
+                         "(DIR/out_<key>.npy), the trained parameters (DIR/param_<i>.npy) or the pulled row_sparse "
+                         "rows (DIR/out_data.npy, DIR/out_indices.npy); float32 (row ids float64), a fixed seeded "
+                         "sample of the larger arrays, 8 Mi elements in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.optimizer is None:
         args.optimizer = "adam" if args.workload == "bert" else "sgd"
     rank = int(os.environ.get("RANK", 0))
@@ -925,9 +974,10 @@ def main():
         numa = bind_to_gpu_numa(local)
         env = Env(args)
         if args.workload == "rsp":
-            res = bench_rsp(env, args)
+            res = bench_rsp(env, args, args.steps, args.dump_outputs)
         else:
-            res = train_steps(env, args, "resnet50" if args.workload == "resnet50-train" else "bert")
+            res = train_steps(env, args, "resnet50" if args.workload == "resnet50-train" else "bert", args.steps,
+                              args.dump_outputs)
         res["numa"] = numa
         if env.rank == 0:
             print(json.dumps(res))
@@ -1017,6 +1067,8 @@ def main():
     host_issue_ms = (time.time() - t_host0) * 1e3 / args.steps      # the host's share: calls are asynchronous
     torch.cuda.synchronize(); env.barrier()
     nvl1 = nvlink_counters(local) if (world > 1 and not args.no_nvml) else None
+    # the untimed steps and the parity check below overwrite `weights`: keep what the last timed step returned
+    snapshot = [w.copyto(ctx) for w in weights] if (args.dump_outputs and rank == 0) else None
     launches = mx.kv.launch_count() - launches0
     variant = variant_since(env, variants0)
     ms_total = ev0.elapsed_time(ev1)
@@ -1126,9 +1178,9 @@ def main():
         secondary = {}
         del kv, grads, weights
         torch.cuda.empty_cache()
-        for name, fn in (("row_sparse_C5", lambda: bench_rsp(env, args)),
-                         ("resnet50_C3", lambda: train_steps(env, args, "resnet50")),
-                         ("bert_base_C4", lambda: train_steps(env, args, "bert"))):
+        for name, fn in (("row_sparse_C5", lambda: bench_rsp(env, args, SECONDARY_RSP_STEPS)),
+                         ("resnet50_C3", lambda: train_steps(env, args, "resnet50", SECONDARY_TRAIN_STEPS)),
+                         ("bert_base_C4", lambda: train_steps(env, args, "bert", SECONDARY_TRAIN_STEPS))):
             try:
                 secondary[name] = fn()
             except Exception as e:          # noqa: BLE001
@@ -1152,6 +1204,8 @@ def main():
             "busbw_gbs_per_gpu": (2.0 * S * (world - 1) / world) / (ms_step * 1e-3) / 1e9 if world > 1 else 0.0,
             "exchange": exchange, "numa": numa,      # (not in `config`: the reference arm prints the same config)
             "sweep": sweep, "secondary": secondary}
+    if snapshot is not None:
+        dump_outputs(args.dump_outputs, [("out_%03d" % k, w.size, w.asnumpy) for k, w in enumerate(snapshot)])
     if parity.get("checked") and not parity.get("ok"):
         sys.stderr.write("PARITY FAILURE: the timed configuration does not match the oracle\n" + json.dumps(line) + "\n")
         env.finish()

@@ -24,9 +24,14 @@
                       mesh of its comments, random matrices of 2 ... 16 GPUs with and without missing links --
                       by Kernighan-Lin and by the exhaustive search; plus the outcome of one Kernighan-Lin pass.
 
+* reference_sums.npz, tree_draw.npz, c_api_prototypes.json -- what the reference's arithmetic, its tree solver and
+                      its C header give for the inputs of three tests that compare with them (see each function).
+
 The GPU box has no /root/reference; tests read the committed fixtures instead.
 """
 import ast
+import hashlib
+import json
 import os
 import sys
 
@@ -449,6 +454,63 @@ def tree_topology():
     print("tree_topology: %d matrices (%d without a tree), %d Kernighan-Lin passes" % (len(cases), fails, len(kl)))
 
 
+def _digest(a):
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), np.uint8)
+
+
+def reference_sums():
+    """The reference's CommDevice / CommCPU sums of the inputs test_dense_sum_against_live_reference_arithmetic draws
+    (seed 5, n = 2 ... 13 values of E elements).  `<kind>_E<E>` [case, i]: the value at idx_E<E>[i] (every element
+    up to 64, a seeded sample above); `<kind>_E<E>_sha256` [case]: the SHA-256 of the whole output, so that the test
+    still compares every bit."""
+    from oracle import oracle as O
+    assert O.ref_lib() is not None, "build oracle/_ref first (make -C oracle)"
+    rng = np.random.default_rng(5)
+    out = {}
+    for n in (2, 3, 4, 5, 6, 8, 9, 13):
+        for E in (1, 17, 5000):
+            idx = out.setdefault("idx_E%d" % E, (np.arange(E) if E <= 64 else np.sort(
+                np.random.default_rng(E).choice(E, 64, replace=False))).astype(np.int64))
+            vals = [rng.uniform(-1, 1, E).astype(np.float32) for _ in range(n)]
+            for kind, s in (("device_f32", O.ref_sum_device(vals)), ("commcpu_f32", O.ref_sum_cpu(vals)),
+                            ("device_f64", O.ref_sum_device([v.astype(np.float64) for v in vals])),
+                            ("device_i32", O.ref_sum_device([(v * 1000).astype(np.int32) for v in vals]))):
+                out.setdefault("%s_E%d" % (kind, E), []).append(s[idx])
+                out.setdefault("%s_E%d_sha256" % (kind, E), []).append(_digest(s))
+    np.savez_compressed(os.path.join(HERE, "reference_sums.npz"), **{k: np.stack(v) if isinstance(v, list) else v
+                                                                     for k, v in out.items()})
+
+
+def tree_draw():
+    """The trees the reference's solver builds for the fixed draw of link matrices in
+    test_trees_match_the_reference_header_compiled_in_place (seed 20260921), case after case: W, alpha, backtrack,
+    and topo / scan, each case's rows of topo_len / scan_len elements, flattened; a case the reference aborts on
+    (no balanced binary tree) has lengths 0."""
+    from oracle import oracle as O
+    assert O.ref_topology_lib() is not None, "build oracle/_ref first (make -C oracle)"
+    sys.path.insert(0, os.path.dirname(HERE))
+    from test_topology import link_matrix_draw
+    cols = {k: [] for k in ("W", "alpha", "backtrack", "topo", "scan", "topo_len", "scan_len")}
+    for W, alpha, bt in link_matrix_draw(np.random.default_rng(20260921)):
+        r = O.ref_compute_trees(W, alpha, bt)
+        topo, scan = (np.zeros((0, 0), np.int16),) * 2 if r is None else (r[0].astype(np.int16), r[1].astype(np.int16))
+        for k, v in (("W", W.ravel()), ("alpha", [alpha]), ("backtrack", [bt]), ("topo", topo.ravel()),
+                     ("scan", scan.ravel()), ("topo_len", [topo.shape[1]]), ("scan_len", [scan.shape[1]])):
+            cols[k].append(np.asarray(v))
+    np.savez_compressed(os.path.join(HERE, "tree_draw.npz"), **{k: np.concatenate(v) for k, v in cols.items()})
+
+
+def c_api_prototypes():
+    """Parameter types of every entry point the reference's include/mxnet/c_api.h declares (test_abi.py::c_prototypes),
+    so that an entry point include/mxkv_b200.h adds later is checked too."""
+    sys.path.insert(0, os.path.dirname(HERE))
+    from test_abi import c_prototypes
+    ref = c_prototypes(os.path.join(REF, "include", "mxnet", "c_api.h"), "MXNET_DLL")
+    with open(os.path.join(HERE, "c_api_prototypes.json"), "w") as f:
+        json.dump(ref, f, indent=1, sort_keys=True)
+        f.write("\n")
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1:                 # e.g. `make_golden.py tree_topology`: only the named fixtures
         for name in sys.argv[1:]:
@@ -461,4 +523,7 @@ if __name__ == "__main__":
     sparse_steps()
     lr_schedules()
     tree_topology()
-    print("wrote", sorted(f for f in os.listdir(HERE) if f.endswith(".npz")))
+    reference_sums()
+    tree_draw()
+    c_api_prototypes()
+    print("wrote", sorted(f for f in os.listdir(HERE) if f.endswith((".npz", ".json"))))

@@ -1,6 +1,7 @@
 """The C-ABI library loads without a GPU and exports every symbol include/mxkv_b200.h declares;
 host-only entry points behave; device entry points fail loudly (no CPU fallback)."""
 import ctypes
+import json
 import os
 import re
 
@@ -389,36 +390,35 @@ def test_engine_defaults_are_the_reference_optimizers():
     assert mx.optimizer.create("adamw").epsilon == 1e-6 and mx.optimizer.create("adam").epsilon == 1e-8
 
 
+def c_prototypes(path, macro):
+    """{entry point: parameter types} of the `macro int name(...);` declarations of a C header."""
+    t = open(path).read()
+    t = re.sub(r"/\*.*?\*/", " ", t, flags=re.S)
+    t = re.sub(r"//[^\n]*", " ", t)
+    out = {}
+    for m in re.finditer(macro + r"\s+int\s+(\w+)\s*\((.*?)\)\s*;", t, flags=re.S):
+        parts = []
+        for a in re.sub(r"DEFAULT\([^)]*\)", "", m.group(2)).split(","):
+            a = " ".join(a.split())
+            if a in ("void", ""):
+                continue
+            if not a.endswith("*"):
+                a = re.sub(r"\s*\b\w+\s*$", "", a)            # drop the parameter name
+            a = a.replace("const ", "").replace(" *", "*").replace("* ", "*").strip()
+            for alias, canon in (("mx_uint", "uint32_t"), ("unsigned int", "uint32_t"), ("dim_t", "int64_t")):
+                a = a.replace(alias, canon)
+            parts.append(a)
+        out[m.group(1)] = parts
+    return out
+
+
 def test_prototypes_match_the_reference_header():
     """Every entry point this library shares with include/mxnet/c_api.h has the reference's parameter types, in
-    order (names and `const` aside; `dim_t` is `int64_t`, `mx_uint` is `uint32_t`).  Needs the reference tree: runs
-    in the authoring container, skips on the GPU box."""
-    ref_h = "/root/reference/include/mxnet/c_api.h"
-    if not os.path.exists(ref_h):
-        pytest.skip("reference tree not present")
-
-    def protos(path, macro):
-        t = open(path).read()
-        t = re.sub(r"/\*.*?\*/", " ", t, flags=re.S)
-        t = re.sub(r"//[^\n]*", " ", t)
-        out = {}
-        for m in re.finditer(macro + r"\s+int\s+(\w+)\s*\((.*?)\)\s*;", t, flags=re.S):
-            parts = []
-            for a in re.sub(r"DEFAULT\([^)]*\)", "", m.group(2)).split(","):
-                a = " ".join(a.split())
-                if a in ("void", ""):
-                    continue
-                if not a.endswith("*"):
-                    a = re.sub(r"\s*\b\w+\s*$", "", a)            # drop the parameter name
-                a = a.replace("const ", "").replace(" *", "*").replace("* ", "*").strip()
-                for alias, canon in (("mx_uint", "uint32_t"), ("unsigned int", "uint32_t"), ("dim_t", "int64_t")):
-                    a = a.replace(alias, canon)
-                parts.append(a)
-            out[m.group(1)] = parts
-        return out
-
-    ref = protos(ref_h, "MXNET_DLL")
-    mine = protos(os.path.join(ROOT, "include", "mxkv_b200.h"), "MXKV_DLL")
+    order (names and `const` aside; `dim_t` is `int64_t`, `mx_uint` is `uint32_t`).  The reference's side is
+    tests/golden/c_api_prototypes.json (make_golden.py::c_api_prototypes)."""
+    with open(os.path.join(ROOT, "tests", "golden", "c_api_prototypes.json")) as f:
+        ref = json.load(f)
+    mine = c_prototypes(os.path.join(ROOT, "include", "mxkv_b200.h"), "MXKV_DLL")
     shared = [n for n in mine if n in ref]
     assert len(shared) >= 50, len(shared)
     for n in shared:

@@ -2,6 +2,7 @@
 golden vectors produced by the reference's own arithmetic / simulators, the reference's
 scenario-level known answers, and an independent restatement of the reference's non-fused
 Python optimizer steps (the reference's own oracle for its fused kernels)."""
+import hashlib
 import os
 
 import numpy as np
@@ -35,18 +36,21 @@ def test_dense_sum_golden_vectors():
     assert np.bitwise_xor.reduce(s.view(np.uint32)) == g["commcpu_f32_big_xor"][0]
 
 
-@pytest.mark.skipif(O.ref_lib() is None, reason="oracle/_ref not built (no /root/reference here)")
 def test_dense_sum_against_live_reference_arithmetic():
+    """tests/golden/reference_sums.npz: what the reference's own arithmetic (oracle/_ref/libkvref.so,
+    make_golden.py::reference_sums) returned for these inputs -- sampled values and the SHA-256 of every output."""
+    g = np.load(os.path.join(GOLD, "reference_sums.npz"))
     rng = np.random.default_rng(5)
-    for n in (2, 3, 4, 5, 6, 8, 9, 13):
+    for case, n in enumerate((2, 3, 4, 5, 6, 8, 9, 13)):
         for E in (1, 17, 5000):
             vals = [rng.uniform(-1, 1, E).astype(np.float32) for _ in range(n)]
-            assert _eq_bits(O.sum_device(vals), O.ref_sum_device(vals))
-            assert _eq_bits(O.sum_cpu(vals), O.ref_sum_cpu(vals))
-            d = [v.astype(np.float64) for v in vals]
-            assert _eq_bits(O.sum_device(d), O.ref_sum_device(d))
-            i = [(v * 1000).astype(np.int32) for v in vals]
-            assert _eq_bits(O.sum_device(i), O.ref_sum_device(i))
+            idx = g["idx_E%d" % E]
+            for kind, s in (("device_f32", O.sum_device(vals)), ("commcpu_f32", O.sum_cpu(vals)),
+                            ("device_f64", O.sum_device([v.astype(np.float64) for v in vals])),
+                            ("device_i32", O.sum_device([(v * 1000).astype(np.int32) for v in vals]))):
+                assert _eq_bits(s[idx], g["%s_E%d" % (kind, E)][case]), (kind, n, E)
+                digest = hashlib.sha256(np.ascontiguousarray(s).tobytes()).digest()
+                assert digest == g["%s_E%d_sha256" % (kind, E)][case].tobytes(), (kind, n, E)
 
 
 def test_compression_golden_vectors():

@@ -4,8 +4,8 @@
 Three pins, strongest first:
 * tests/golden/tree_topology.npz: trees the reference's compiled header produced for 136 link matrices (one
   switch, the NVLink cube mesh, random 2 ... 16 GPUs; Kernighan-Lin and exhaustive search) -- always checked;
-* oracle/_ref/libkvref_topo.so, the reference header compiled in place: random matrices (a fixed draw; fresh ones in soak runs), when the
-  library is there (authoring container; it travels to the GPU box prebuilt);
+* oracle/_ref/libkvref_topo.so, the reference header compiled in place: random matrices -- a fixed draw against the
+  trees it returned, stored in tests/golden/tree_draw.npz; fresh ones in soak runs, when the library is there;
 * the known answers of the reference's unit test, tests/cpp/kvstore/gpu_topology_test.cc, function by function.
 Then the derived add schedules: the kernel's own evaluator (csrc/tree_math.h compiled for the host) against the
 oracle's level-by-level restatement of CommDeviceTree::ReduceInner on every golden tree."""
@@ -54,11 +54,8 @@ def test_kernighan_lin_pass_matches_the_reference_golden(golden):
         assert [int(v) for p in pairs for v in p] == golden["kl_%d_pairs" % i].tolist()
 
 
-@pytest.mark.skipif(O.ref_topology_lib() is None, reason="oracle/_ref/libkvref_topo.so not built (no /root/reference)")
-def test_trees_match_the_reference_header_compiled_in_place():
-    # a fixed draw in the gating suite; MXKV_FUZZ_SEEDS > 0 (soak runs): fresh matrices every time
-    fresh = int(os.environ.get("MXKV_FUZZ_SEEDS", "0")) > 0
-    rng = np.random.default_rng(int.from_bytes(os.urandom(4), "little") if fresh else 20260921)
+def link_matrix_draw(rng):
+    """(W, alpha, backtrack) for random link matrices of 2 ... 16 GPUs, some with missing links."""
     for n in (2, 3, 4, 5, 6, 7, 8, 9, 11, 13, 16):
         for rep in range(3):
             u = rng.uniform(0, 1, (n, n))
@@ -69,13 +66,40 @@ def test_trees_match_the_reference_header_compiled_in_place():
             W = (W + W.T).astype(np.float32)
             alpha = float(rng.choice([0.7, 0.5, 0.9]))
             for bt in ((False, True) if n <= 5 else (False,)):
-                want = O.ref_compute_trees(W, alpha, bt)
-                if want is None:
-                    with pytest.raises(mx.MXNetError):
-                        T.compute_trees(W, alpha, bt)
-                    continue
-                topo, scan, _ = T.compute_trees(W, alpha, bt)
-                assert np.array_equal(topo, want[0]) and np.array_equal(scan, want[1]), (n, rep, bt, W.tolist())
+                yield W, alpha, bt
+
+
+def test_trees_match_the_reference_header_compiled_in_place():
+    """A fixed draw against tests/golden/tree_draw.npz (what oracle/_ref/libkvref_topo.so returned for it,
+    make_golden.py::tree_draw); MXKV_FUZZ_SEEDS > 0 (soak runs): fresh matrices against that library itself."""
+    fresh = int(os.environ.get("MXKV_FUZZ_SEEDS", "0")) > 0
+    if fresh and O.ref_topology_lib() is None:
+        pytest.skip("fresh matrices need oracle/_ref/libkvref_topo.so (built by oracle/Makefile from the reference tree)")
+    gold = None if fresh else dict(np.load(os.path.join(HERE, "golden", "tree_draw.npz")))
+    rng = np.random.default_rng(int.from_bytes(os.urandom(4), "little") if fresh else 20260921)
+    at = dict.fromkeys(("W", "topo", "scan"), 0)
+
+    def take(name, count):
+        at[name] += count
+        return gold[name][at[name] - count:at[name]]
+
+    i = -1
+    for i, (W, alpha, bt) in enumerate(link_matrix_draw(rng)):
+        n = W.shape[0]
+        if fresh:
+            want = O.ref_compute_trees(W, alpha, bt)
+        else:
+            assert np.array_equal(W.ravel(), take("W", n * n)), i
+            assert alpha == gold["alpha"][i] and bt == gold["backtrack"][i], i
+            tl, sl = int(gold["topo_len"][i]), int(gold["scan_len"][i])
+            want = (take("topo", n * tl).reshape(n, tl), take("scan", n * sl).reshape(n, sl)) if tl else None
+        if want is None:
+            with pytest.raises(mx.MXNetError):
+                T.compute_trees(W, alpha, bt)
+            continue
+        topo, scan, _ = T.compute_trees(W, alpha, bt)
+        assert np.array_equal(topo, want[0]) and np.array_equal(scan, want[1]), (i, bt, W.tolist())
+    assert fresh or (i + 1 == gold["alpha"].size and at["W"] == gold["W"].size and at["topo"] == gold["topo"].size)
 
 
 # ---- tests/cpp/kvstore/gpu_topology_test.cc, case by case -------------------------------------------------------
